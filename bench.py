@@ -91,6 +91,27 @@ class ClockSampler:
                 "samples": len(self.rows), "power_w_max": max(pw) if pw else None}
 
 
+DUMP_PARAM_SAMPLE = 4 << 20   # trainable parameters written by --dump-outputs (16 MB of float32)
+
+
+def dump_outputs(out_dir, ps, loss):
+    """What the last timed step hands its caller, as .npy files: the loss (float64), the L2 norm of every trainable parameter
+    tensor after the update (float64, named_parameters order) and a fixed seeded sample of DUMP_PARAM_SAMPLE trainable
+    parameter values (float32, positions in the concatenation of those tensors, ascending).  Inputs and initial weights are
+    seeded, but the split-K weight gradients are summed with atomic adds in whatever order the CTAs finish, so two runs agree
+    to float rounding, not bit for bit: compare with a tolerance."""
+    import torch
+    module = ps.module if hasattr(ps, "module") else ps.model
+    params = [p.detach() for p in module.parameters() if p.requires_grad]
+    flat = torch.cat([p.reshape(-1).float() for p in params])
+    idx = np.unique(np.random.default_rng(0).integers(0, flat.numel(), size=min(flat.numel(), DUMP_PARAM_SAMPLE)))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array(loss, np.float64))
+    np.save(os.path.join(out_dir, "param_norms.npy"),
+            torch.stack([torch.linalg.vector_norm(p.double()) for p in params]).cpu().numpy())
+    np.save(os.path.join(out_dir, "param_sample.npy"), flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy())
+
+
 def cpu_threads():
     """Threads for the CPU arm: every core up to 32 (beyond that the small ops of the step only get slower)."""
     return min(os.cpu_count() or 1, 32)
@@ -288,7 +309,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="run the step eagerly instead of replaying the captured CUDA graph")
     ap.add_argument("--no-kernel-rooflines", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="training-step workloads: after the timed steps, write what the last one computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload.startswith("pointops")):
+        ap.error("--dump-outputs needs --impl b200 and a training-step workload (gps_pretrain, scanrefer, objcls)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -473,6 +500,8 @@ def main():
 
     with ClockSampler(local_rank) as cs:
         total_ms, launches, loss = timed(step_resident, args.steps, warmup)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, ps, loss)   # before the e2e steps below move the parameters on
         e2e_ms, _, _ = timed(step_e2e, args.steps, warmup)
     clocks = cs.summary()
     ms_per_step = total_ms / args.steps

@@ -1,10 +1,12 @@
-"""ORACLE — TEST INFRASTRUCTURE ONLY.  Run ON THE GPU BOX:  python oracle/make_golden_gpu.py
+"""ORACLE — TEST INFRASTRUCTURE ONLY.  Run on a B200:  python oracle/make_golden_gpu.py OUT_DIR
 
-Runs the REFERENCE's own CUDA kernels (oracle/_ref/_ext_ref.so = /root/reference's
+Runs the REFERENCE's own CUDA kernels (oracle/_ref/_ext_ref.so = the reference's
 _ext_src/src/*.cu compiled for sm_100a by oracle/build_ref_ext.py) on seeded inputs and writes
-small .npz fixtures (inputs + reference outputs) to gpurun_out/golden/; they are then committed
-under tests/golden/ and pin both the CPU oracle (tests/test_oracle.py) and the CUDA library
-(tests/test_pointops_gpu.py).  It also cross-checks the CPU oracle on every case it writes.
+small .npz fixtures to OUT_DIR; they are then committed under tests/golden/:
+  * pointops_*.npz (inputs + reference outputs) pin both the CPU oracle (tests/test_oracle.py) and the
+    CUDA library (tests/test_pointops_gpu.py).  The CPU oracle is cross-checked on every one of them.
+  * reference_cuda_cases.npz: reference outputs only, for the seeded inputs of tests/cases.py that
+    tests/test_pointops_gpu.py compares bit for bit (a seeded sample of rows of the largest ball queries).
 """
 import os
 import sys
@@ -22,11 +24,33 @@ def dev(a):
     return torch.from_numpy(np.ascontiguousarray(a)).cuda()
 
 
-def main():
+def reference_cuda_cases(ref, out):
+    z = {}
+    for name, (xyz, m) in {**cases.fps_cases(), **cases.fps_cases_large()}.items():
+        z["fps__" + name] = ref.furthest_point_sampling(dev(xyz), m).cpu().numpy()
+    for name, (new_xyz, xyz, r, ns) in cases.bq_cases().items():
+        z["bq__" + name] = ref.ball_query(dev(new_xyz), dev(xyz), r, ns).cpu().numpy()
+    for j, (u, k, _, _, _) in enumerate(cases.three_nn_cases()):
+        d, i = ref.three_nn(dev(u), dev(k))
+        z[f"three_nn__{j}__dist2"], z[f"three_nn__{j}__idx"] = d.cpu().numpy(), i.cpu().numpy()
+    for B, N in cases.SWEEP_SHAPES:
+        xyz, m, r = cases.sweep_case(B, N)
+        x = dev(xyz)
+        idx = ref.furthest_point_sampling(x, m)
+        cen = torch.gather(x, 1, idx.long()[..., None].expand(-1, -1, 3)).contiguous()
+        bq = ref.ball_query(cen, x, r, 32).cpu().numpy().reshape(B * m, 32)
+        rows = np.sort(np.random.default_rng(0).choice(B * m, size=min(B * m, 1024), replace=False))
+        z[f"sweep__{B}x{N}__fps"] = idx.cpu().numpy()
+        z[f"sweep__{B}x{N}__bq_rows"], z[f"sweep__{B}x{N}__bq"] = rows, bq[rows]
+    np.savez_compressed(os.path.join(out, "reference_cuda_cases.npz"), **z)
+    print("reference_cuda_cases:", len(z), "arrays,", sum(v.nbytes for v in z.values()), "bytes")
+
+
+def main(out):
     ref = build_ref_ext.load_prebuilt()
     assert ref is not None, "oracle/_ref/_ext_ref.so missing"
-    out = os.path.join(ROOT, "gpurun_out", "golden")
     os.makedirs(out, exist_ok=True)
+    reference_cuda_cases(ref, out)
     bad = 0
     fps = cases.fps_cases()
     keep = ["sa1_objects", "sa2_shape", "ball_n3", "ball_n80", "ball_n100", "ball_n513", "ball_n1000",
@@ -85,4 +109,4 @@ def main():
 
 
 if __name__ == "__main__":
-    sys.exit(1 if main() else 0)
+    sys.exit(1 if main(sys.argv[1]) else 0)

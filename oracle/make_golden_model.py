@@ -153,11 +153,30 @@ def golden_gps_backward():
     print("backward golden:", float(total), len(norms), "parameter gradients")
 
 
+def golden_qa_head():
+    """QAHeadV1 (modules/heads/qa_head.py) with name-keyed synthetic weights (seed 11) on seeded object / text features."""
+    import importlib
+    ref = importlib.import_module("modules.heads.qa_head").QAHeadV1(None, num_answers=200).eval()
+    ref.load_state_dict(weights.synthetic_state_dict(ref, seed=11))
+    g = torch.Generator().manual_seed(0)
+    obj, txt = torch.randn(3, 20, 768, generator=g), torch.randn(3, 12, 768, generator=g)
+    om = torch.rand(3, 20, generator=g) > 0.3
+    om[:, 0] = True
+    tm = torch.arange(12)[None, :] < torch.tensor([12, 5, 9])[:, None]
+    with torch.no_grad():
+        out = ref(obj, om, txt, tm)
+    shapes = json.dumps({k: list(v.shape) for k, v in ref.state_dict().items()})
+    np.savez_compressed(os.path.join(OUT, "model_qa_head.npz"), weight_seed=11, input_seed=0, state_dict_shapes=shapes,
+                        out=out.numpy())
+    print("qa head golden:", tuple(out.shape))
+
+
 def main():
     ref_shims.install()
     torch.manual_seed(0)
     golden_gps_stack()
     golden_gps_backward()
+    golden_qa_head()
     shapes = {"PointNetPP": golden_pointnetpp()}
     # state_dict contracts of the registry classes (SURVEY.md §8b): key -> shape
     from modules.build import GROUNDING_REGISTRY, HEADS_REGISTRY, VISION_REGISTRY

@@ -12,6 +12,7 @@ tensors, so that the unmodified reference Python layers can run on CPU with
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -22,9 +23,16 @@ _lib = None
 
 
 def build(force=False):
-    """gcc -O2 -ffp-contract=off -fopenmp; returns the .so path."""
+    """gcc -O2 -ffp-contract=off -fopenmp; returns the .so path.  It goes to oracle/_build, or to a fresh temporary
+    directory when that cannot be written (a read-only checkout)."""
+    global _OUT
     if force or not os.path.exists(_OUT) or os.path.getmtime(_OUT) < os.path.getmtime(_SRC):
-        os.makedirs(os.path.dirname(_OUT), exist_ok=True)
+        try:
+            os.makedirs(os.path.dirname(_OUT), exist_ok=True)
+        except OSError:
+            pass
+        if not os.access(os.path.dirname(_OUT), os.W_OK):
+            _OUT = os.path.join(tempfile.mkdtemp(prefix="svref-"), "libsvref.so")
         tmp = _OUT + ".%d.tmp" % os.getpid()
         subprocess.check_call(
             ["gcc", "-O2", "-ffp-contract=off", "-fopenmp", "-shared", "-fPIC", "-o", tmp, _SRC, "-lm"])

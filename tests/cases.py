@@ -35,6 +35,29 @@ def fps_cases_large():
     return cases
 
 
+def three_nn_cases():
+    """[(unknown (B,n,3), known (B,m,3), feats (B,c,m), weight (B,n,3), grad_out (B,c,n))], one seeded stream"""
+    rng = np.random.default_rng(1)
+    out = []
+    for (B, n, m, c) in [(2, 300, 64, 8), (1, 17, 2, 3), (2, 1024, 2500, 4)]:
+        u = rng.standard_normal((B, n, 3)).astype(np.float32)
+        k = rng.standard_normal((B, m, 3)).astype(np.float32)
+        feats = rng.standard_normal((B, c, m)).astype(np.float32)
+        w = rng.random((B, n, 3)).astype(np.float32)
+        g = rng.standard_normal((B, c, n)).astype(np.float32)
+        out.append((u, k, feats, w, g))
+    return out
+
+
+# BASELINE.json configs[4] shapes: (batch, points); m = N/32, r = 0.2 (1024/N)^(1/3), nsample 32
+SWEEP_SHAPES = [(2, 16384), (1, 65536), (1, 262144)]
+
+
+def sweep_case(B, N):
+    """(xyz (B,N,3), m, radius) of one sweep shape"""
+    return synthetic.unit_ball_clouds(11, B, N), N // 32, float(0.2 * (1024.0 / N) ** (1.0 / 3.0))
+
+
 def bq_cases():
     """name -> (new_xyz (B,M,3), xyz (B,N,3), radius, nsample)"""
     rng = np.random.default_rng(3)

@@ -1,6 +1,7 @@
 """GPU parity tests of libsvpointops (through the `_ext` drop-in, i.e. through the C-ABI) against
-the CPU oracle, bit-exact for index work, and — when oracle/_ref is present — against the
-reference's own CUDA kernels compiled for sm_100a."""
+the CPU oracle, bit-exact for index work, and against the reference's own CUDA kernels compiled for
+sm_100a: their stored outputs on the same seeded inputs (tests/golden/reference_cuda_cases.npz, made by
+oracle/make_golden_gpu.py) and, when oracle/_ref is present, the kernels themselves."""
 import glob
 import os
 
@@ -20,6 +21,11 @@ def ext():
     return _ext
 
 
+@pytest.fixture(scope="module")
+def ref_golden():
+    return np.load(os.path.join(GOLDEN, "reference_cuda_cases.npz"))
+
+
 def dev(a):
     return torch.from_numpy(np.ascontiguousarray(a)).cuda()
 
@@ -28,21 +34,23 @@ ALL_FPS = {**cases.fps_cases(), **cases.fps_cases_large()}
 
 
 @pytest.mark.parametrize("name", sorted(ALL_FPS))
-def test_fps_bit_exact(ext, oracle, ref_ext, name):
+def test_fps_bit_exact(ext, oracle, ref_ext, ref_golden, name):
     xyz, m = ALL_FPS[name]
     got = ext.furthest_point_sampling(dev(xyz), m).cpu().numpy()
     want = oracle.furthest_point_sampling(xyz, m)
     np.testing.assert_array_equal(got, want, err_msg=f"vs oracle: {name}")
+    np.testing.assert_array_equal(got, ref_golden["fps__" + name], err_msg=f"vs reference CUDA golden: {name}")
     if ref_ext is not None:
         ref = ref_ext.furthest_point_sampling(dev(xyz), m).cpu().numpy()
         np.testing.assert_array_equal(got, ref, err_msg=f"vs reference CUDA: {name}")
 
 
 @pytest.mark.parametrize("name", sorted(cases.bq_cases()))
-def test_ball_query_bit_exact(ext, oracle, ref_ext, name):
+def test_ball_query_bit_exact(ext, oracle, ref_ext, ref_golden, name):
     new_xyz, xyz, r, ns = cases.bq_cases()[name]
     got = ext.ball_query(dev(new_xyz), dev(xyz), r, ns).cpu().numpy()
     np.testing.assert_array_equal(got, oracle.ball_query(new_xyz, xyz, r, ns), err_msg=f"vs oracle: {name}")
+    np.testing.assert_array_equal(got, ref_golden["bq__" + name], err_msg=f"vs reference CUDA golden: {name}")
     if ref_ext is not None:
         ref = ref_ext.ball_query(dev(new_xyz), dev(xyz), r, ns).cpu().numpy()
         np.testing.assert_array_equal(got, ref, err_msg=f"vs reference CUDA: {name}")
@@ -109,23 +117,20 @@ def test_group_gather_exact_and_grads(ext, oracle):
                                    oracle.gather_points_grad(g2, i2, N), rtol=1e-5, atol=1e-5)
 
 
-def test_three_nn_interpolate(ext, oracle, ref_ext):
-    rng = np.random.default_rng(1)
-    for (B, n, m, c) in [(2, 300, 64, 8), (1, 17, 2, 3), (2, 1024, 2500, 4)]:
-        u = rng.standard_normal((B, n, 3)).astype(np.float32)
-        k = rng.standard_normal((B, m, 3)).astype(np.float32)
+def test_three_nn_interpolate(ext, oracle, ref_ext, ref_golden):
+    for j, (u, k, feats, w, g) in enumerate(cases.three_nn_cases()):
+        m = k.shape[1]
         d, i = ext.three_nn(dev(u), dev(k))
         wd, wi = oracle.three_nn(u, k)
         np.testing.assert_array_equal(i.cpu().numpy(), wi)
         np.testing.assert_array_equal(d.cpu().numpy(), wd)
+        np.testing.assert_array_equal(i.cpu().numpy(), ref_golden[f"three_nn__{j}__idx"])
+        np.testing.assert_array_equal(d.cpu().numpy(), ref_golden[f"three_nn__{j}__dist2"])
         if ref_ext is not None:
             rd, ri = ref_ext.three_nn(dev(u), dev(k))
             assert torch.equal(ri, i) and torch.equal(rd, d)
-        feats = rng.standard_normal((B, c, m)).astype(np.float32)
-        w = rng.random((B, n, 3)).astype(np.float32)
         out = ext.three_interpolate(dev(feats), dev(wi), dev(w)).cpu().numpy()
         np.testing.assert_array_equal(out, oracle.three_interpolate(feats, wi, w))
-        g = rng.standard_normal(out.shape).astype(np.float32)
         np.testing.assert_allclose(ext.three_interpolate_grad(dev(g), dev(wi), dev(w), m).cpu().numpy(),
                                    oracle.three_interpolate_grad(g, wi, w, m), rtol=1e-4, atol=1e-4)
 
@@ -202,14 +207,13 @@ def test_batches_beyond_the_grid_y_limit():
     assert torch.equal(_ext.gather_points(pts, gi), torch.gather(pts, 2, gi.long()[:, None].expand(-1, 2, -1)))
 
 
-@pytest.mark.parametrize("B,N", [(2, 16384), (1, 65536), (1, 262144)])
-def test_sweep_shapes_bit_exact_against_the_reference_cuda_kernels(ext, oracle, ref_ext, B, N):
+@pytest.mark.parametrize("B,N", cases.SWEEP_SHAPES)
+def test_sweep_shapes_bit_exact_against_the_reference_cuda_kernels(ext, oracle, ref_ext, ref_golden, B, N):
     """BASELINE.json configs[4] shapes (16 K - 256 K points, m = N/32, r = 0.2 (1024/N)^(1/3), nsample 32): FPS (multi-CTA path for
-    N > 8192) and ball query bit-exact against the reference's own CUDA kernels (oracle/_ref); the CPU oracle covers the 16 K and
-    64 K cases (its FPS is O(N m))."""
-    from sceneverse_b200 import synthetic
-    xyz = synthetic.unit_ball_clouds(11, B, N)
-    m, r = N // 32, float(0.2 * (1024.0 / N) ** (1.0 / 3.0))
+    N > 8192) and ball query bit-exact against the reference's own CUDA kernels (their stored FPS indices and a seeded sample of
+    1024 ball-query rows; all of it against oracle/_ref when present); the CPU oracle covers the 16 K and 64 K cases (its FPS is
+    O(N m))."""
+    xyz, m, r = cases.sweep_case(B, N)
     x = dev(xyz)
     idx = ext.furthest_point_sampling(x, m)
     cen = torch.gather(x, 1, idx.long()[..., None].expand(-1, -1, 3)).contiguous()
@@ -218,6 +222,9 @@ def test_sweep_shapes_bit_exact_against_the_reference_cuda_kernels(ext, oracle, 
         want_i = oracle.furthest_point_sampling(xyz, m)
         np.testing.assert_array_equal(idx.cpu().numpy(), want_i)
         np.testing.assert_array_equal(bq.cpu().numpy(), oracle.ball_query(cen.cpu().numpy(), xyz, r, 32))
+    key = f"sweep__{B}x{N}__"
+    np.testing.assert_array_equal(idx.cpu().numpy(), ref_golden[key + "fps"])
+    np.testing.assert_array_equal(bq.cpu().numpy().reshape(B * m, 32)[ref_golden[key + "bq_rows"]], ref_golden[key + "bq"])
     if ref_ext is not None:
         np.testing.assert_array_equal(idx.cpu().numpy(), ref_ext.furthest_point_sampling(x, m).cpu().numpy())
         np.testing.assert_array_equal(bq.cpu().numpy(), ref_ext.ball_query(cen, x, r, 32).cpu().numpy())
