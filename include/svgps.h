@@ -115,10 +115,14 @@ int sv_attention_fwd_lse_bf16(const void *q, long long q_bs, int q_rs, const voi
                               const unsigned char *key_padding_mask, const float *spatial_w, int spatial_heads,
                               const float *pairwise_locs, int B, int H, int Lq, int Lk, float scale, float *lse,
                               void *stream);
-/* Backward of the fused attention (one tcgen05 kernel template launched twice: dQ + gate-weight gradients with tile rows
- * == queries, dK/dV with tile rows == keys; both recompute P from Q, K, the gate and lse).  q/k/v as in the forward; o, d_o (B,Lq,H*64) bf16
- * contiguous; dq (B,Lq,H*64), dk, dv (B,Lk,H*64) bf16 contiguous; d_spatial_w (B,Lq,H*6) f32 (NULL without gate; gate
- * requires spatial_heads == H); dvec (B,H,Lq) f32 scratch.  Lq, Lk <= 384. */
+/* Backward of the fused attention; P is recomputed from Q, K, the gate and lse.  Without the gate ONE tcgen05 kernel (tile
+ * rows == keys) computes P and dS once per (query, key) pair and produces dQ, dK and dV; keys past the last unmasked one
+ * are skipped (their dK / dV rows are written as zeros).  With the gate two launches: dQ + gate-weight gradients with tile
+ * rows == queries, dK/dV with tile rows == keys.  q/k/v as in the forward; o, d_o (B,Lq,H*64) bf16 contiguous; dq
+ * (B,Lq,H*64), dk, dv (B,Lk,H*64) bf16 contiguous; d_spatial_w (B,Lq,H*6) f32 (NULL without gate; gate requires
+ * spatial_heads == H); dvec: f32 scratch of sv_attention_bwd_scratch_floats(B, H, Lq, Lk) floats ((B,H,Lq) up to 128
+ * keys, (B,H,Lq,64) beyond: the dQ partial sums over the key tiles).  Lq, Lk <= 384. */
+int sv_attention_bwd_scratch_floats(int B, int H, int Lq, int Lk);
 int sv_attention_bwd_bf16(const void *q, long long q_bs, int q_rs, const void *k, long long k_bs, int k_rs,
                           const void *v, long long v_bs, int v_rs, const void *o, const void *d_o,
                           const unsigned char *key_padding_mask, const float *spatial_w, const float *pairwise_locs,

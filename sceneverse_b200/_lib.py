@@ -99,6 +99,7 @@ _GPS_SIGS = {
                                       ctypes.c_longlong, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                       c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
                                       c_void_p, c_float, ctypes.c_ulonglong, c_void_p],
+    "sv_attention_bwd_scratch_floats": [c_int, c_int, c_int, c_int],
     "sv_layer_norm_fwd": [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_float, ctypes.c_ulonglong,
                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
     "sv_layer_norm_bwd": [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_float, ctypes.c_ulonglong,

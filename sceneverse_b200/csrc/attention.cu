@@ -13,6 +13,9 @@
 // P goes back to shared memory as the K-major A operand of O = P V, whose B operand is the SAME staged V tile read
 // MN-major (no transposed copy).  O reuses the TMEM columns of S.  All loops over keys are rolled 16-column units, so
 // the kernel body stays inside the instruction cache.
+// Keys past the last unmasked one of the scene (`kend`, from the key-padding mask) are skipped: the S MMA, the softmax
+// units and the P V k-steps stop at round16(kend).  Their weights are exactly 0, so the output and lse are bit-identical
+// to the same scene with those keys cut off.
 #include "attn_common.cuh"
 #include "svgps.h"
 
@@ -55,6 +58,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap mq, const __grid_constant__ 
   float *xsum = xmax + 256;                  // [2][128] per-warpgroup row sums
   uint64_t *bars = reinterpret_cast<uint64_t *>(xsum + 256);  // 0: K/V landed, 1: Q tile landed, 2: MMA done
   uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 3);
+  int *kend_s = reinterpret_cast<int *>(tmem_slot + 1);        // 1 + index of the last unmasked key
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, wg = warp >> 2, wq = warp & 3;
   const int row = wq * 32 + lane;            // tile row == TMEM lane of this thread
@@ -65,6 +69,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap mq, const __grid_constant__ 
     mbar_init(&bars[1], 1);
     mbar_init(&bars[2], 1);
     mbar_fence_init();
+    *kend_s = 0;
     tma_prefetch_desc(&mq);
     tma_prefetch_desc(&mk);
     tma_prefetch_desc(&mv);
@@ -78,15 +83,23 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap mq, const __grid_constant__ 
     tma_rows(sQ, &mq, h, 0, 8, a.Lq, b, &bars[1]);
   }
   if (warp == 1) tmem_alloc_n(tmem_slot, a.tmem_cols);
-  for (int j = tid; j < 384; j += 256)
-    kb[j] = (j < a.Lk && !(a.kpm != nullptr && a.kpm[(size_t)b * a.Lk + j])) ? 0.f : -INFINITY;
+  int last = 0;
+  for (int j = tid; j < 384; j += 256) {
+    const bool live = j < a.Lk && !(a.kpm != nullptr && a.kpm[(size_t)b * a.Lk + j]);
+    kb[j] = live ? 0.f : -INFINITY;
+    if (live) last = j + 1;
+  }
+  last = __reduce_max_sync(0xffffffffu, last);
+  if (lane == 0 && last > 0) atomicMax(kend_s, last);
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
   const uint32_t tmem = *tmem_slot;
   const uint32_t trow = tmem + ((uint32_t)(wq * 32) << 16);
   const float c2 = a.scale * LOG2E;
-  const int nu = NK >> 4;                    // 16-column units, split between the two warpgroups
+  // keys swept: round16(kend), at least one unit so that a scene with every key masked still gets O = 0 from P V
+  const int NKe = max(16, (*kend_s + 15) & ~15);
+  const int nu = NKe >> 4;                   // 16-column units, split between the two warpgroups
   const int u_begin = wg == 0 ? 0 : (nu + 1) / 2, u_end = wg == 0 ? (nu + 1) / 2 : nu;
   const bool vec_loc = GATED && (a.Lk & 3) == 0;
   uint32_t ph_q = 0, ph_m = 0;
@@ -101,8 +114,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap mq, const __grid_constant__ 
       mbar_wait(&bars[1], ph_q);
       fence_after_sync();
       const uint32_t aQ = smem_u32(sQ), aK = smem_u32(sK);
-      for (int n0 = 0; n0 < NK; n0 += 256) {  // one MMA covers at most 256 keys
-        const uint32_t idesc = idesc_kk(min(256, NK - n0));
+      for (int n0 = 0; n0 < NKe; n0 += 256) {  // one MMA covers at most 256 keys
+        const uint32_t idesc = idesc_kk(min(256, NKe - n0));
 #pragma unroll
         for (int ks = 0; ks < DH / 16; ++ks)
           mma_bf16_e(tmem + n0, make_desc_sw128(aQ + ks * 32), make_desc_sw128(aK + n0 * 128 + ks * 32), idesc, ks > 0);

@@ -86,20 +86,20 @@ def attention_backward(q, k, v, out, grad_out, lse, num_heads, key_padding_mask=
         dk = torch.empty((B, Lk, E), dtype=torch.bfloat16, device=dev)
         dv = torch.empty((B, Lk, E), dtype=torch.bfloat16, device=dev)
         d_rs = E
-    dvec = torch.empty((B, num_heads, Lq), dtype=torch.float32, device=dev)
+    lib = _lib.gps()
+    scratch = torch.empty(lib.sv_attention_bwd_scratch_floats(B, num_heads, Lq, Lk), dtype=torch.float32, device=dev)
     kpm = _mask_bytes(key_padding_mask)
     sw = locs = dsw = None
     if spatial_w is not None:
         sw, locs = spatial_w.float().contiguous(), pairwise_locs.float().contiguous()
         dsw = torch.empty_like(sw)
-    lib = _lib.gps()
     with torch.cuda.device(dev):
         st = lib.sv_attention_bwd_strided_bf16(
             q.data_ptr(), q.stride(0), q.stride(1), k.data_ptr(), k.stride(0), k.stride(1), v.data_ptr(), v.stride(0),
             v.stride(1), out.data_ptr(), grad_out.data_ptr(), kpm.data_ptr() if kpm is not None else None,
             sw.data_ptr() if sw is not None else None, locs.data_ptr() if locs is not None else None, lse.data_ptr(),
             B, num_heads, Lq, Lk, 0.125, dq.data_ptr(), dk.data_ptr(), dv.data_ptr(), d_rs,
-            dsw.data_ptr() if dsw is not None else None, dvec.data_ptr(), float(dropout_p), int(seed),
+            dsw.data_ptr() if dsw is not None else None, scratch.data_ptr(), float(dropout_p), int(seed),
             torch.cuda.current_stream(dev).cuda_stream)
     _lib.check(lib, st, "sv_attention_bwd_strided_bf16")
     return dq, dk, dv, dsw
